@@ -94,6 +94,24 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+# ------------------------------------------------------------------------------------------------ output dump
+DUMP_BUDGET = 60 * 2 ** 20          # bytes of array data; with the .npy headers the dump stays under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes `arrays` (name -> float32 / float64 numpy array) as out_dir/<name>.npy, so that two builds run with the same
+    arguments can be compared output for output. Above DUMP_BUDGET in all, every array is cut to its share of the budget by
+    a fixed, seeded sample of its flattened elements (ascending indices, the same in every run with the same arguments)."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        if total > DUMP_BUDGET:
+            idx = np.random.default_rng(0).choice(a.size, a.size * DUMP_BUDGET // total, replace=False)
+            a = a.reshape(-1)[np.sort(idx)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------ workloads
 def make_state_dicts(C, G):
     """Seeded parameters for the two networks (reference key names / shapes)."""
@@ -402,6 +420,10 @@ def run_ours(args, emit):
         out_holder["seg"], out_holder["cont"] = pred.predict(feat_dev)
     ms_unet = timed(unet_step, args.steps, args.warmup)
     pred.seg_network.check(); pred.cont_network.check()
+    dump = {}                                                                       # what the last timed step returned
+    if args.dump_outputs and rank == 0:
+        dump["unet_seg_logits"] = out_holder["seg"].float().cpu().numpy()
+        dump["unet_cont_pred"] = out_holder["cont"].float().cpu().numpy()
 
     # ---- region 2: MPM rollout, state resident; every step restarts from the same initial scene
     solver = setup_solver(sc, ng, dev)
@@ -416,6 +438,11 @@ def run_ours(args, emit):
     ms_mpm = timed(mpm_step, args.steps, args.warmup, prep=mpm_prep)
     mpm_launches_per_rollout = (solver.launch_count() - launches0) / (args.steps + args.warmup)
     x_after_rollout = solver.export_particle_x_to_torch().clone()                   # state after SUB substeps from the initial scene
+    if args.dump_outputs and rank == 0:
+        for name, t in (("x", solver.export_particle_x_to_torch()), ("v", solver.export_particle_v_to_torch()),
+                        ("F", solver.export_particle_F_to_torch()), ("C", solver.export_particle_C_to_torch()),
+                        ("stress", solver.export_particle_stress_to_torch())):
+            dump[f"mpm_{name}"] = t.float().cpu().numpy()
     clocks = sampler.stop() if rank == 0 else None
 
     # ---- optional variants of SURVEY 8d config 3: the SVD-based plastic materials (one rollout each, after a warm-up)
@@ -551,6 +578,8 @@ def run_ours(args, emit):
         dist.destroy_process_group()
     if rank != 0:
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dump)
     K = args.steps
     vps = world * G ** 3 * K / (ms_unet * 1e-3)
     pps = world * n * SUB * K / (ms_mpm * 1e-3)
@@ -606,7 +635,11 @@ def main():
     ap.add_argument("--slab-migrate-every", type=int, default=25, help="substeps between two migration check points")
     ap.add_argument("--slab-lazy-trigger", type=int, default=2,
                     help="migrate only once a particle is this many planes outside its slab (0: migrate at every check point)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed U-Net and MPM steps returned in their last step as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the outputs of --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     # the shims mirror the reference's progress prints; keep stdout for the ONE JSON line
