@@ -175,7 +175,6 @@ conv3d_igemm_kernel(const __grid_constant__ ConvKernelParams p) {
     if (warp == 0) {
         // ================================================================ TMA producer (warp-uniform, one elected lane issues)
         int ws = 0, wph = 0, ss = 0, sph = 0;
-        int wcount = 0, scount = 0;     // bring-up only (debug_flags bit 1: stop re-loading once every stage was filled)
         bool ok = true;
         for (int wi = blockIdx.x; wi < total_items && ok; wi += gridDim.x) {
             const TileCoord t = decode_tile(p, wi);
@@ -184,15 +183,13 @@ conv3d_igemm_kernel(const __grid_constant__ ConvKernelParams p) {
                 const int ntaps = P.n_kh * P.n_kd;
                 ok = mbar_wait(&ctl->wempty[ws], wph ^ 1, abort_flag);
                 if (!ok) break;
-                if ((p.debug_flags & 2) && wcount >= p.w_stages) { if (elect_one()) mbar_arrive(&ctl->wfull[ws]); }
-                else if (elect_one()) {
+                if (elect_one()) {
                     mbar_expect_tx(&ctl->wfull[ws], (uint32_t)(ntaps * p.block_n * 128));
                     uint8_t* wdst = w_smem + (size_t)ws * p.w_stage_bytes;
                     for (int tap = 0; tap < ntaps; ++tap)
                         tma_load_2d(wdst + (size_t)tap * p.block_n * 128, &p.tmB, &ctl->wfull[ws],
                                     (P.wtile_base + tap) * 64, t.n0);
                 }
-                ++wcount;
                 if (++ws == p.w_stages) { ws = 0; wph ^= 1; }
 
                 const int nplanes = t.tde + P.n_kd - 1;
@@ -200,14 +197,12 @@ conv3d_igemm_kernel(const __grid_constant__ ConvKernelParams p) {
                 for (int pl = 0; pl < nplanes && ok; ++pl) {
                     ok = mbar_wait(&ctl->sempty[ss], sph ^ 1, abort_flag);
                     if (!ok) break;
-                    if ((p.debug_flags & 2) && scount >= p.s_stages) { if (elect_one()) mbar_arrive(&ctl->sfull[ss]); }
-                    else if (elect_one()) {
+                    if (elect_one()) {
                         mbar_expect_tx(&ctl->sfull[ss], slab_bytes);
                         tma_load_5d(s_smem + (size_t)ss * p.s_stage_bytes, &p.tmA[P.src],
                                     &ctl->sfull[ss], (int)P.c0, t.w0 * p.stride + P.dw,
                                     t.h0 * p.stride + P.dh0, (t.d0 + pl) * p.stride + P.dd0, t.nb);
                     }
-                    ++scount;
                     if (++ss == p.s_stages) { ss = 0; sph ^= 1; }
                 }
             }
@@ -224,7 +219,7 @@ conv3d_igemm_kernel(const __grid_constant__ ConvKernelParams p) {
                        idesc3_h = make_idesc_f16(128, (uint32_t)(3 * p.block_n));
         const uint32_t idesc1_q = make_idesc_e5m2(128, (uint32_t)p.block_n), idesc2_q = make_idesc_e5m2(128, (uint32_t)(2 * p.block_n)),
                        idesc3_q = make_idesc_e5m2(128, (uint32_t)(3 * p.block_n));
-        const uint64_t desc_fixed = (make_sw128_desc(0, 1024) ^ p.desc_xor);   // everything but the start address
+        const uint64_t desc_fixed = make_sw128_desc(0, 1024);   // everything but the start address
         const uint32_t desc_lo = (uint32_t)desc_fixed, desc_hi = (uint32_t)(desc_fixed >> 32);
         const bool fast3 = (p.block_n == 64 || p.block_n == 128) && (p.TW == 16 || p.TW == 8);
         const uint32_t w_base0 = smem_u32(w_smem), s_base0 = smem_u32(s_smem);
@@ -325,30 +320,14 @@ conv3d_igemm_kernel(const __grid_constant__ ConvKernelParams p) {
         bool ok = true;
         const long long DHW = (long long)p.D * p.H * p.W;
         const bool do_stats = p.stats != nullptr;
-        const bool scalar_stats = do_stats && p.stats_scalar;     // consumer only needs the per-item totals (LayerNorm)
         float* my_stats = stats_sm + (size_t)(warp - 2) * 2 * stats_ld;
         const int et = threadIdx.x - 64;        // 0..127 among the epilogue threads
         int stats_nb = -1;
-        double tot_s = 0.0, tot_q = 0.0;        // scalar mode: this thread's running totals
-        if (do_stats && !scalar_stats) {
+        if (do_stats) {
             for (int i = lane; i < 2 * stats_ld; i += 32) my_stats[i] = 0.f;
             __syncwarp();
         }
         auto flush_stats = [&](int nb) {
-            if (scalar_stats) {
-                // totals go to channel 0's slot; the LayerNorm consumer sums the [Cout][2] row anyway
-#pragma unroll
-                for (int off = 16; off >= 1; off >>= 1) {
-                    tot_s += __shfl_xor_sync(0xffffffffu, tot_s, off);
-                    tot_q += __shfl_xor_sync(0xffffffffu, tot_q, off);
-                }
-                if (lane == 0) {
-                    atomicAdd(p.stats + (size_t)nb * p.Cout * 2, tot_s);
-                    atomicAdd(p.stats + (size_t)nb * p.Cout * 2 + 1, tot_q);
-                }
-                tot_s = 0.0; tot_q = 0.0;
-                return;
-            }
             // all 4 epilogue warps: fold the warp-private partial sums into the global fp64 accumulators
             asm volatile("bar.sync 1, 128;" ::: "memory");
             for (int ch = et; ch < p.Cout; ch += 128) {
@@ -370,13 +349,6 @@ conv3d_igemm_kernel(const __grid_constant__ ConvKernelParams p) {
             float sq[16];
 #pragma unroll
             for (int j = 0; j < 16; ++j) sq[j] = f[j] * f[j];
-            if (scalar_stats) {
-                float s = 0.f, q2 = 0.f;
-#pragma unroll
-                for (int j = 0; j < 16; ++j) { s += f[j]; q2 += sq[j]; }
-                tot_s += (double)s; tot_q += (double)q2;
-                return;
-            }
             const float s1 = warp_colsum16(f, lane);
             const float s2 = warp_colsum16(sq, lane);
             const int chn = ch0 + stats_channel_of_lane(lane);
@@ -389,7 +361,7 @@ conv3d_igemm_kernel(const __grid_constant__ ConvKernelParams p) {
         const bool wide_ok = !p.out_planar && ((p.out_ld & 3) == 0) && ((p.out_c0 & 3) == 0);
         // 256-bit accesses need 32-byte aligned rows (cudaMalloc'ed bases are 256-byte aligned)
         const bool wide8_ok = wide_ok && ((p.out_ld & 7) == 0) && ((p.out_c0 & 7) == 0) && ((reinterpret_cast<uintptr_t>(p.out) & 31) == 0) &&
-                              (p.residual == nullptr || (reinterpret_cast<uintptr_t>(p.residual) & 31) == 0) && !(p.debug_flags & 8);
+                              (p.residual == nullptr || (reinterpret_cast<uintptr_t>(p.residual) & 31) == 0);
         for (int wi = blockIdx.x; wi < total_items && ok; wi += gridDim.x) {
             const TileCoord t = decode_tile(p, wi);
             ok = mbar_wait(&ctl->tfull[as], aph, abort_flag);
@@ -408,7 +380,7 @@ conv3d_igemm_kernel(const __grid_constant__ ConvKernelParams p) {
             // the warp ONCE per (tile, chunk): the per-plane shuffle reduction cost 10 % of a 64->64 conv (r01) and its
             // 250 shuffles per plane competed with the MMA issuer for the MIO queue.
             int c_wide = 0;
-            if (wide_ok && !(p.debug_flags & 1)) {
+            if (wide_ok) {
                 const bool use_bias = first_split && p.bias != nullptr;
                 const bool use_res = row_ok && first_split && p.residual != nullptr;
                 const long long plane_ld = (long long)p.H * p.W * p.out_ld;
@@ -488,22 +460,15 @@ conv3d_igemm_kernel(const __grid_constant__ ConvKernelParams p) {
                         if (two) finish(v1, r1, base0 + plane_ld);
                     }
                     if (do_stats) {
-                        if (scalar_stats) {
-                            float s = 0.f, q2 = 0.f;
-#pragma unroll
-                            for (int j = 0; j < 32; ++j) { s += cs[j]; q2 += cq[j]; }
-                            tot_s += (double)s; tot_q += (double)q2;
-                        } else {
-                            const float s1 = warp_colsum32(cs, lane);       // lane l ends up with channel ch0 + l
-                            const float s2 = warp_colsum32(cq, lane);
-                            my_stats[ch0 + lane] += s1;
-                            my_stats[stats_ld + ch0 + lane] += s2;
-                            __syncwarp();
-                        }
+                        const float s1 = warp_colsum32(cs, lane);       // lane l ends up with channel ch0 + l
+                        const float s2 = warp_colsum32(cq, lane);
+                        my_stats[ch0 + lane] += s1;
+                        my_stats[stats_ld + ch0 + lane] += s2;
+                        __syncwarp();
                     }
                 }
             }
-            for (int d = 0; d < t.tde && !(p.debug_flags & 1); ++d) {
+            for (int d = 0; d < t.tde; ++d) {
                 const long long vox = ((long long)(t.d0 + d) * p.H + hh) * p.W + ww;   // inside batch item
                 const uint32_t acc = tmem_base + ((uint32_t)(q * 32) << 16) +
                                      (uint32_t)((as * p.TD + d) * p.block_n);
@@ -884,10 +849,6 @@ int conv_plan_create(const ConvDesc& d, int* d_err_flag, ConvPlan& plan, char* e
     p.out_ld = d.out_ld ? d.out_ld : d.Cout; p.out_c0 = d.out_c0; p.out_planar = d.out_planar;
     p.err_flag = d_err_flag;
     p.stats = plan.fused_stats ? d.stats : nullptr;
-    p.stats_scalar = d.stats_scalar ? 1 : 0;
-    p.desc_xor = 0;
-    p.debug_flags = 0;
-    if (const char* e = getenv("PIXIE_CONV_DEBUG")) p.debug_flags = atoi(e);    // bring-up A/B switches (see conv3d_igemm.cuh)
     plan.out_bytes = d.out_planar ? (size_t)d.NB * d.Cout * d.D * d.H * d.W * 4
                                   : (size_t)d.NB * d.D * d.H * d.W * p.out_ld * 4;
 

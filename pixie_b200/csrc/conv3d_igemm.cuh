@@ -77,12 +77,7 @@ struct ConvKernelParams {
                              // accumulated by the epilogue (fused LayerNorm/GroupNorm statistics); or nullptr
     int stats_ld;            // floats per statistics row in shared memory (Cout rounded up to 32)
     int smem_slack;          // bytes reserved for aligning the dynamic smem base to 1 KB (0: the base must already be aligned)
-    int stats_scalar;        // 1: only the per-item totals are wanted; they land in channel 0's slot (LayerNorm consumers)
     int* err_flag;           // device int, set non-zero on pipeline timeout
-    uint64_t desc_xor;       // bring-up only: xor into every smem matrix descriptor (0 in product use)
-    int debug_flags;         // bring-up only, timing experiments (results are WRONG when set): 1 = epilogue skips its body,
-                             // 2 = producer stops issuing TMA once every stage was filled; 8 = epilogue uses 128-bit instead of
-                             // 256-bit global accesses (results stay correct)
 };
 
 // One activation source of a convolution.
@@ -114,7 +109,6 @@ struct ConvDesc {
     float* out = nullptr;
     int out_ld = 0, out_c0 = 0, out_planar = 0;
     double* stats = nullptr;           // request fused output statistics (honoured iff plan.fused_stats)
-    bool stats_scalar = false;         // totals only (see ConvKernelParams::stats_scalar)
     int split_k = 1;                   // >1 => atomics into pre-zeroed out
     int block_n = 0;                   // 0 = choose
     int td = 0;                        // 0 = choose

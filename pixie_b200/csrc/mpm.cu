@@ -202,7 +202,6 @@ struct Mpm {
     int ov_lo[2] = {0, 0}, ov_hi[2] = {0, 0};
     bool g2p_pending = false;          // slab phases: the gather of the last finished substep has not run yet
     float slab_dt = 0.f;               // ... and the dt it has to use
-    int agg = 2;                       // log2 of the longest aggregated run in the scatter: PIXIE_MPM_AGG; r02 sweep: 1 and 2 tie at 100k/64^3 and at 1M/256^3, 0 is 10-15 % slower at both
     long long launches = 0;            // kernels of this library launched for this handle (bench.py's gpu_launches)
 };
 
@@ -366,13 +365,12 @@ int mpm_sync(Mpm* m, cudaStream_t st) {
 // (or captured graph) is still draining; both kernels of the substep chain wait for it with griddepcontrol.wait.
 template <typename... KArgs, typename... Args>
 static void pdl_launch(void (*kern)(KArgs...), dim3 grid, dim3 block, cudaStream_t st, Args... args) {
-    static const bool pdl = !(getenv("PIXIE_MPM_PDL") && atoi(getenv("PIXIE_MPM_PDL")) == 0);
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = 0; cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = pdl ? 1 : 0;
+    cfg.attrs = attr; cfg.numAttrs = 1;
     cudaLaunchKernelEx(&cfg, kern, KArgs(args)...);
 }
 
@@ -420,13 +418,8 @@ static void fused_launch(Mpm* m, bool do_g2p, bool do_p2g, bool write_all, float
     t.do_g2p = do_g2p; t.do_p2g = do_p2g; t.write_all = write_all;
     t.time = m->tslots + m->tpar;                 // clock of the substep whose stress / scatter runs in this launch
     // 88 registers per thread: 32-thread blocks pack 23 per SM (736 threads), so 100k particles are one wave on 148 SMs
-    static const int B = [] { const char* e = getenv("PIXIE_MPM_FUSED_BLOCK"); const int b = e ? atoi(e) : kFusedThreads; return (b == 32 || b == 64 || b == 128) ? b : kFusedThreads; }();
-    const int blocks = (std::max(m->n_active, 1) + B - 1) / B;
-    static const bool hoist = !(getenv("PIXIE_MPM_HOIST") && atoi(getenv("PIXIE_MPM_HOIST")) == 0);   // r02 A/B: 23.5 vs 24.1 us
-    void (*kern)(const FusedState, const float) = mpm_fused_kernel<2, false>;
-    if (hoist) kern = m->agg == 0 ? mpm_fused_kernel<0, true> : (m->agg == 1 ? mpm_fused_kernel<1, true> : (m->agg == 3 ? mpm_fused_kernel<3, true> : mpm_fused_kernel<2, true>));
-    else kern = m->agg == 0 ? mpm_fused_kernel<0, false> : (m->agg == 1 ? mpm_fused_kernel<1, false> : (m->agg == 3 ? mpm_fused_kernel<3, false> : mpm_fused_kernel<2, false>));
-    pdl_launch(kern, dim3(blocks), dim3(B), st, t, dt);
+    const int blocks = (std::max(m->n_active, 1) + kFusedThreads - 1) / kFusedThreads;
+    pdl_launch(mpm_fused_kernel, dim3(blocks), dim3(kFusedThreads), st, t, dt);
     m->launches += 1;
 }
 
@@ -554,7 +547,6 @@ Mpm* mpm_create(int n_particles, int n_grid, float grid_lim, std::string& err) {
     cudaMemset(m->grid_v, 0, nodes * sizeof(float4));
     cudaMemset(m->tslots, 0, 2 * sizeof(double));
     cudaMemset(m->pts, 0, (size_t)2 * kMaxBC * 3 * sizeof(float));
-    if (const char* a = getenv("PIXIE_MPM_AGG")) m->agg = std::min(3, std::max(0, atoi(a)));
     return m;
 }
 

@@ -16,7 +16,7 @@
 //     instead of ~35).  Same arithmetic, different association: results agree with the reference order to fp32
 //     rounding (tests/test_mpm_golden.py holds both to the reference-generated vectors);
 //   * the scatter is warp-aggregated like before (runs of equal base cell, segmented shuffle, one red.global.add.v4.f32
-//     per run and node), with the run length a template parameter.
+//     per run of up to 4 lanes and node).
 // Included by mpm.cu inside its anonymous namespace (DevBC, M3/V3, the constitutive functions).
 // Reference statements restated: mpm_utils.py:338-463 (p2g, g2p), 467-526 (stress), 583-588 (damping);
 // mpm_solver_warp.py:528-547 (particle BCs), :785-974 (grid BCs), :899-905 + :637 (moving cuboid, clock).
@@ -234,12 +234,6 @@ __device__ __forceinline__ bool any_particle_bc_active(const FusedState& s, floa
     return any;
 }
 
-// AGG = log2 of the longest run of equal-cell lanes that is summed before one red is issued (0: no aggregation)
-__device__ __forceinline__ void prefetch_l1(const void* p) { asm volatile("prefetch.global.L1 [%0];" ::"l"(p)); }
-
-// HOIST: issue the late-needed per-particle loads at the top (costs registers across the gather); otherwise only prefetch
-// their lines into L1 there and load at the point of use
-template <int AGG, bool HOIST>
 __global__ void __maxnreg__(88)
 mpm_fused_kernel(const __grid_constant__ FusedState s, const float dt) {
     // programmatic dependent launch: let the next kernel of the chain get scheduled while this one runs, and wait here
@@ -257,26 +251,19 @@ mpm_fused_kernel(const __grid_constant__ FusedState s, const float dt) {
     const bool act = live && s.selection[p] == 0;
     const int n = s.n_grid;
 
-    // every load whose address is known up front is issued here, back to back: with ~5 warps per scheduler each dependent
-    // trip to L2 that is taken alone costs the warp ~300 idle cycles (r02 ncu: 40 % of the stall samples were long-scoreboard)
+    // every load whose address is known up front is issued here, back to back, although the values are needed only after
+    // the gather (costs registers across it): with ~5 warps per scheduler each dependent trip to L2 that is taken alone
+    // costs the warp ~300 idle cycles (r02 ncu: 40 % of the stall samples were long-scoreboard)
     float px = f[(FS_X + 0) * cap + p], py = f[(FS_X + 1) * cap + p], pz = f[(FS_X + 2) * cap + p];
-    float mass, vol, mu, lam, time = 0.f;
-    int material, orig = 0;
+    const float mass = f[FS_MASS * cap + p], vol = f[FS_VOL * cap + p];
+    float mu = f[FS_MU * cap + p], lam = f[FS_LAM * cap + p];
+    const int material = s.material[p];
+    float time = 0.f;
+    int orig = 0;
+    if (s.n_particle_bc > 0) { orig = s.perm[p]; time = (float)(*s.time); }
     int box[6];
-    auto late_loads = [&]() {
-        mass = f[FS_MASS * cap + p]; vol = f[FS_VOL * cap + p];
-        mu = f[FS_MU * cap + p]; lam = f[FS_LAM * cap + p];
-        material = s.material[p];
-        if (s.n_particle_bc > 0) { orig = s.perm[p]; time = (float)(*s.time); }
 #pragma unroll
-        for (int k = 0; k < 6; ++k) box[k] = s.box[k];
-    };
-    if (HOIST) late_loads();
-    else if ((threadIdx.x & 31) == 0) {           // one lane per warp pulls the warp's lines (128 B = 32 particles) into L1
-        prefetch_l1(f + FS_MASS * cap + p); prefetch_l1(f + FS_VOL * cap + p); prefetch_l1(f + FS_MU * cap + p);
-        prefetch_l1(f + FS_LAM * cap + p); prefetch_l1(s.material + p); prefetch_l1(s.box);
-        if (s.n_particle_bc > 0) prefetch_l1(s.perm + p);
-    }
+    for (int k = 0; k < 6; ++k) box[k] = s.box[k];
     float vx, vy, vz;
     M3 C, Ft;
 
@@ -339,7 +326,6 @@ mpm_fused_kernel(const __grid_constant__ FusedState s, const float dt) {
     }
 
     // ---------------------------------------------------------------------- particle BCs, stress (substep i+1)
-    if (!HOIST) late_loads();
     if (s.n_particle_bc > 0 && any_particle_bc_active(s, time)) {
         const bool dirty = particle_bcs(s, orig, time, dt, mass, px, py, pz, vx, vy, vz);
         // the reference stores the modified v; only particles outside the selection keep it (g2p overwrites the rest)
@@ -410,28 +396,24 @@ mpm_fused_kernel(const __grid_constant__ FusedState s, const float dt) {
         atomicMax(s.box + 3, min(max(ax.b, 0), n - 3) + 3); atomicMax(s.box + 4, min(max(ay.b, 0), n - 3) + 3); atomicMax(s.box + 5, min(max(az.b, 0), n - 3) + 3);
     }
 
-    // runs of equal base cell among consecutive lanes, chopped at 2^AGG lanes
+    // runs of equal base cell among consecutive lanes, chopped at 4 lanes and summed in two segmented-shuffle levels
+    // (aggregation depth from the r02 sweep, DESIGN 4.3)
     const unsigned full = 0xffffffffu;
     const int lane = threadIdx.x & 31;
     const bool contrib = act;
     const int key = (contrib && inside) ? (ax.b * n + ay.b) * n + az.b : -1 - lane;      // odd particles never share a run
-    bool head = true;
-    bool c1 = false, c2 = false, c4 = false;
-    if (AGG > 0) {
-        const int kprev = __shfl_up_sync(full, key, 1);
-        head = (lane == 0) || (key != kprev);
-        unsigned H = __ballot_sync(full, head);
-        const int hl = 31 - __clz(H & (0xffffffffu >> (31 - lane)));      // head lane of my run
-        head = head || (((lane - hl) & ((1 << AGG) - 1)) == 0);
-        H = __ballot_sync(full, head);
-        const unsigned above = H & ~((2u << lane) - 1u);                   // heads strictly above this lane
-        const int seg_end = above ? (__ffs(above) - 2) : 31;               // last lane of my segment
-        c1 = lane + 1 <= seg_end; c2 = lane + 2 <= seg_end; c4 = lane + 4 <= seg_end;
-    }
+    const int kprev = __shfl_up_sync(full, key, 1);
+    bool head = (lane == 0) || (key != kprev);
+    unsigned H = __ballot_sync(full, head);
+    const int hl = 31 - __clz(H & (0xffffffffu >> (31 - lane)));          // head lane of my run
+    head = head || (((lane - hl) & 3) == 0);
+    H = __ballot_sync(full, head);
+    const unsigned above = H & ~((2u << lane) - 1u);                       // heads strictly above this lane
+    const int seg_end = above ? (__ffs(above) - 2) : 31;                   // last lane of my segment
+    const bool c1 = lane + 1 <= seg_end, c2 = lane + 2 <= seg_end;
     auto segsum = [&](float v) {
-        if (AGG >= 1) { const float t = __shfl_down_sync(full, v, 1); if (c1) v += t; }
-        if (AGG >= 2) { const float t = __shfl_down_sync(full, v, 2); if (c2) v += t; }
-        if (AGG >= 3) { const float t = __shfl_down_sync(full, v, 4); if (c4) v += t; }
+        float t = __shfl_down_sync(full, v, 1); if (c1) v += t;
+        t = __shfl_down_sync(full, v, 2); if (c2) v += t;
         return v;
     };
 

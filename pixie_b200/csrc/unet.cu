@@ -78,7 +78,7 @@ struct UNet {
     static constexpr int kGraphSlots = 4;
     GraphEntry graphs[kGraphSlots];
     int graph_next = 0;
-    bool use_graph = true;
+    bool use_graph = true;          // cleared when a capture or instantiation fails: launch directly from then on
 
     ~UNet() {
         for (auto& g : graphs) if (g.exec) cudaGraphExecDestroy(g.exec);
@@ -470,7 +470,6 @@ UNet* unet_create(const pixie_unet_config& cfg, std::string& err) {
     if (cfg.precision < 0 || cfg.precision > 2) { err = "precision must be 0 (fp16), 1 (fp16x3) or 2 (fp16 + e5m2 corrections)"; return nullptr; }
     auto* u = new UNet();
     u->cfg = cfg;
-    u->use_graph = getenv("PIXIE_NO_GRAPH") == nullptr;
     u->NBmax = cfg.max_batch > 0 ? cfg.max_batch : 1;
     return u;
 }

@@ -334,13 +334,12 @@ int launch_pack_predictions(const float* seg, const float* cont, float* out, int
 // The convolution kernel runs with the maximum shared-memory carve-out (222 KB per CTA). A kernel that asks for the default
 // split makes the SM re-partition L1 / shared memory at the kernel boundary, which it can only do when idle; the streaming
 // kernels here do not need L1, so they ask for the same carve-out and the ~390 launches of a network keep one configuration.
-// PIXIE_UNET_CARVEOUT=0 restores the default (A/B switch).
-template <typename K>
-static inline void prefer_max_smem_carveout(K kernel) {
-    static const bool on = !(getenv("PIXIE_UNET_CARVEOUT") && atoi(getenv("PIXIE_UNET_CARVEOUT")) == 0);
-    if (on) cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
+// The attribute is set once per kernel, before its first launch.
+template <auto kernel>
+static inline void prefer_max_smem_carveout() {
+    static const cudaError_t set = cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
+    (void)set;
 }
-#define PIXIE_CARVEOUT_ONCE(kernel) do { static bool done_ = false; if (!done_) { prefer_max_smem_carveout(kernel); done_ = true; } } while (0)
 
 // Voxels per block: one trip of a block covers (256 / (C/4)) * 4 voxel rows; aim at >= 2 blocks per SM so that the
 // 16^3 and 8^3 levels are not run by 16 blocks (r01 ncu: 20 us for a 2 MB tensor), capped at 512 voxels for the big levels.
@@ -355,7 +354,7 @@ int launch_moments(const float* x, int NB, int V, int C, double* stats, cudaStre
     if (C % 4 || C / 4 > 256) return 1;
     const int vpb = vox_per_block_for(V, C);
     dim3 grid((V + vpb - 1) / vpb, NB);
-    PIXIE_CARVEOUT_ONCE(moments_kernel);
+    prefer_max_smem_carveout<moments_kernel>();
     moments_kernel<<<grid, 256, 0, st>>>(x, V, C, vpb, stats);
     return (int)cudaGetLastError();
 }
@@ -366,9 +365,9 @@ int launch_norm_act(NormArgs a, int NB, cudaStream_t st) {
     dim3 grid((a.V + a.vox_per_block - 1) / a.vox_per_block, NB);
     const int lom = !a.dst_lo ? 2 : (a.lo_mode == 1 ? 1 : 0);
 #define PIXIE_NORM_L(M, A) \
-    do { if (lom == 2) { PIXIE_CARVEOUT_ONCE((norm_act_kernel<M, A, 2>)); norm_act_kernel<M, A, 2><<<grid, 256, 0, st>>>(a); } \
-         else if (lom == 1) { PIXIE_CARVEOUT_ONCE((norm_act_kernel<M, A, 1>)); norm_act_kernel<M, A, 1><<<grid, 256, 0, st>>>(a); } \
-         else { PIXIE_CARVEOUT_ONCE((norm_act_kernel<M, A, 0>)); norm_act_kernel<M, A, 0><<<grid, 256, 0, st>>>(a); } } while (0)
+    do { if (lom == 2) { prefer_max_smem_carveout<norm_act_kernel<M, A, 2>>(); norm_act_kernel<M, A, 2><<<grid, 256, 0, st>>>(a); } \
+         else if (lom == 1) { prefer_max_smem_carveout<norm_act_kernel<M, A, 1>>(); norm_act_kernel<M, A, 1><<<grid, 256, 0, st>>>(a); } \
+         else { prefer_max_smem_carveout<norm_act_kernel<M, A, 0>>(); norm_act_kernel<M, A, 0><<<grid, 256, 0, st>>>(a); } } while (0)
 #define PIXIE_NORM_A(M) \
     do { if (a.act == kActSiLU) PIXIE_NORM_L(M, kActSiLU); else if (a.act == kActLeaky) PIXIE_NORM_L(M, kActLeaky); else PIXIE_NORM_L(M, kActNone); } while (0)
     if (a.mode == kNormLN) PIXIE_NORM_A(kNormLN);
@@ -381,7 +380,7 @@ int launch_norm_act(NormArgs a, int NB, cudaStream_t st) {
 
 int launch_upsample2(const float* x, __half* y, __half* ylo, int lo_mode, int NB, int sp, int C, cudaStream_t st) {
     const long long total4 = (long long)NB * 8 * sp * sp * sp * (C / 4);
-    PIXIE_CARVEOUT_ONCE(upsample2_kernel);
+    prefer_max_smem_carveout<upsample2_kernel>();
     upsample2_kernel<<<(unsigned)((total4 + 255) / 256), 256, 0, st>>>(x, y, ylo, lo_mode, sp, C, total4);
     return (int)cudaGetLastError();
 }
@@ -390,7 +389,7 @@ int launch_attention(const float* qkv, __half* out, __half* out_lo, int lo_mode,
     const size_t smem = (size_t)kAttnQ * (C + T) * sizeof(float);
     if (smem > 48 * 1024 || C % 4) return 1;
     dim3 grid((T + kAttnQ - 1) / kAttnQ, NB);
-    PIXIE_CARVEOUT_ONCE(attention_kernel);
+    prefer_max_smem_carveout<attention_kernel>();
     attention_kernel<<<grid, 256, smem, st>>>(qkv, out, out_lo, lo_mode, T, C);
     return (int)cudaGetLastError();
 }

@@ -1,5 +1,6 @@
-"""MPM timing A/B on the GPU box (BASELINE config 3: 100k particles, 64^3 grid): the default path with each scatter
-aggregation depth (the round-1 four-kernel path it replaced measured 46.6 us on the same box, profiles/r02_mpm_fused_first_perf.log). Usage: python scripts/gpu_mpm_perf.py [substeps]"""
+"""MPM timing on the GPU box (BASELINE config 3: 100k particles, 64^3 grid): the default scene, the same without BCs, and
+(mode "full") a sand scene and 1M particles on 128^3 (the round-1 four-kernel path the fused one replaced measured 46.6 us on
+the same box, profiles/r02_mpm_fused_first_perf.log). Usage: python scripts/gpu_mpm_perf.py [substeps] [full|quick]"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -43,21 +44,7 @@ def time_it(tag, steps, **kw):
 if __name__ == "__main__":
     steps = int(sys.argv[1]) if len(sys.argv) > 1 else 1000
     mode = sys.argv[2] if len(sys.argv) > 2 else "full"
-    if mode == "ab":          # same-box A/B of the launch / load-placement variants (each process-wide switch is read once per process)
-        import subprocess
-        for hoist in ("0", "1"):
-            for pdl in ("1", "0"):
-                env = dict(os.environ, PIXIE_MPM_HOIST=hoist, PIXIE_MPM_PDL=pdl)
-                out = subprocess.run([sys.executable, __file__, str(steps), "one"], env=env, capture_output=True, text=True).stdout
-                print(f"hoist={hoist} pdl={pdl}: " + " | ".join(l for l in out.splitlines() if "us/substep" in l), flush=True)
-        sys.exit(0)
-    if mode == "one":
-        time_it("fused", steps)
-        sys.exit(0)
-    for agg in ((2, 3, 1) if mode == "full" else (2,)):
-        os.environ["PIXIE_MPM_AGG"] = str(agg)
-        time_it(f"fused agg={agg}", steps)
-    os.environ["PIXIE_MPM_AGG"] = "2"
+    time_it("fused", steps)
     time_it("fused, no BCs", steps, bcs=False)
     if mode == "full":
         time_it("fused, sand", steps, materials=(2,))
